@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- decode tokens/s + p50 per-token latency of the MoE dispatch hot path, Mixtral-8x7B shapes.
 
-Contract (see task statement): `python bench.py --gpus N --steps K --warmup W [--impl reference]`
-prints ONE JSON line on rank 0.
+Usage: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]`
+prints ONE JSON line on rank 0.  --dump-outputs DIR (single-GPU Mixtral path) writes DIR/out.npy: the float32 copy of the
+[layers, 8, 4096] hidden states the last timed step returned; the inputs are seeded, so two builds can be compared output for
+output.  Nothing is written into the source tree.
 
 Workload (N=1, BASELINE.json configs[1]): Mixtral-8x7B bf16, random-init N(0,0.02^2) weights, 32 MoE layers,
 8 experts, top-2, H=4096, I=14336; decode batch 8 => T=8 tokens enter every MoE block per step; all 256
@@ -35,6 +37,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "moe-infinity_b200")):
     if p not in sys.path:
@@ -295,6 +298,14 @@ def algorithmic_bytes(counts_per_layer, T, cfg):
     return total, k3
 
 
+def dump_outputs(directory, **arrays):
+    """What the timed path returned in its last step, as float32 .npy files (one per name)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     from moe_infinity_b200 import MoEEngine
@@ -365,6 +376,8 @@ def run_ours(args):
         evs[i + 1].record()
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out=out_dev)
     step_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     total_ms = evs[0].elapsed_time(evs[-1])
     ms_per_step = total_ms / args.steps
@@ -673,8 +686,11 @@ def run_deepseek(args):
         _view(p.value, (3 * Hh * 2 * I,), dtype, eng.device).normal_(0, 0.02)
         eng._ck(eng.lib.b2m_register_shared(eng._h, l, None, 0))
     peak, peak_src = load_peaks()
-    with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
-        tf_peak = float(json.load(f).get("bf16_tflops_sustained", 1417.8))
+    tf_peak, tf_src = 1417.8, "fallback (no MEASURED_PEAKS.json)"
+    if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")):
+        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
+            tf_peak = float(json.load(f).get("bf16_tflops_sustained", tf_peak))
+        tf_src = "measured (MEASURED_PEAKS.json bf16_tflops_sustained)"
 
     def measure(T, iters, graph=True):
         x = torch.randn(Lr, T, Hh, device=dev).to(dtype)
@@ -741,12 +757,12 @@ def run_deepseek(args):
 
     sampler = ClockSampler(0)
     sampler.start()
-    dec = measure(16, max(args.steps, 10))
+    dec = measure(16, args.steps)
     clocks = sampler.stop()
     pre = measure(Tp, 3, graph=False) if Tp > 0 else None
     line = {
         "metric": "decode tokens/sec + p50 per-token latency, DeepSeek-V2-Lite MoE dispatch path", "value": dec["tokens_per_s"],
-        "unit": "tokens/s", "n_gpus": 1, "steps": max(args.steps, 10), "warmup": 2, "ms_per_step": dec["ms_per_step"],
+        "unit": "tokens/s", "n_gpus": 1, "steps": args.steps, "warmup": 2, "ms_per_step": dec["ms_per_step"],
         "p50_token_latency_ms": dec["p50_ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
         "data": "synthetic",
         "config": {"workload": f"DeepSeek-V2-Lite MoE dispatch path: {Lr} MoE layers x 64 routed experts top-6 + 2 shared, H=2048 "
@@ -759,10 +775,10 @@ def run_deepseek(args):
                      "algorithmic_bytes_per_step": dec["algorithmic_bytes"]},
         "e2e": {"value": dec["e2e_tokens_per_s"], "unit": "tokens/s", "h2d_bytes_per_step": dec["h2d_bytes"],
                 "d2h_bytes_per_step": dec["d2h_bytes"], "ms_per_step": dec["e2e_ms_per_step"]},
-        "gpu_launches": int(dec["launches_per_step"] * max(args.steps, 10)), "clocks": clocks, "decode": dec,
+        "gpu_launches": int(dec["launches_per_step"] * args.steps), "clocks": clocks, "decode": dec,
         "prefill": None if pre is None else dict(pre, roofline={"bound": "tensor", "achieved": pre["tflops"], "peak": tf_peak,
                                                                "unit": "TFLOP/s", "frac": pre["tensor_frac"],
-                                                               "peak_source": "measured (MEASURED_PEAKS.json bf16_tflops_sustained)"}),
+                                                               "peak_source": tf_src}),
     }
     print(json.dumps(line), flush=True)
 
@@ -785,7 +801,13 @@ def main():
     ap.add_argument("--layers", type=int, default=0, help="debug: fewer layers (invalid as a bench value)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float32; single-GPU mixtral path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "mixtral" or args.gpus != 1):
+        ap.error("--dump-outputs covers the single-GPU mixtral path (--config mixtral --gpus 1 --impl ours)")
     if args.impl == "reference":
         return run_reference(args)
     if not torch.cuda.is_available():

@@ -1,8 +1,7 @@
-"""CPU: host policy code -- tracer/predictor/prefetcher mirrors against the LITERAL reference classes
-(/root/reference/moe_infinity/memory/*.py, dev container only) and the cache-policy oracle's stated rules."""
-import contextlib
+"""CPU: host policy code -- tracer/predictor/prefetcher mirrors against what the LITERAL reference classes
+(moe_infinity/memory/*.py of the reference) computed on the same seeded inputs (tests/golden/reference_results.pt, written by
+tests/golden/make_reference_golden.py), and the cache-policy oracle's stated rules."""
 import os
-import types
 
 import numpy as np
 import pytest
@@ -10,80 +9,39 @@ import torch
 
 from moe_infinity_b200 import memory as M
 from oracle.policy_oracle import CacheOracle
+from reference_cases import PREDICTOR_SEEDS, PRIORITY_LAYERS, library, prefetch_inputs, priority_inputs
 
-HAVE_REF = os.path.isdir("/root/reference/moe_infinity/memory")
-
-
-@contextlib.contextmanager
-def _cpu_only_torch():
-    """The literal ExpertTracer allocates on cuda:0 (expert_tracer.py:33-35,104); run it on CPU."""
-    zeros, to = torch.zeros, torch.Tensor.to
-
-    def zeros_cpu(*a, **k):
-        k.pop("device", None)
-        return zeros(*a, **k)
-
-    def to_cpu(self, *a, **k):
-        if any(isinstance(x, str) and x == "cpu" for x in a):
-            return self.clone()      # cuda:0 -> cpu is a copy in the real run; keep that (the caller mutates it)
-        a = tuple(x for x in a if not (isinstance(x, str) and x.startswith("cuda")))
-        if not a and not k:
-            return self
-        return to(self, *a, **k)
-
-    torch.zeros, torch.Tensor.to = zeros_cpu, to_cpu
-    try:
-        yield
-    finally:
-        torch.zeros, torch.Tensor.to = zeros, to
+REF = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_results.pt"),
+                 weights_only=False)["memory"]
 
 
-def _cfg(L, E):
-    return types.SimpleNamespace(architectures=["MixtralForCausalLM"], num_hidden_layers=L, num_local_experts=E)
-
-
-def _library(rng, n, L, E):
-    lib = rng.integers(0, 6, size=(n, L, E)).astype(np.float32)
-    lib[:, :, 0] += 1.0   # no all-zero rows
-    return lib
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("seed", [0, 1, 2])
+@pytest.mark.parametrize("seed", PREDICTOR_SEEDS)
 def test_predictor_matches_literal_reference(seed):
-    import ref_loader
-    ns = ref_loader.load()
+    ref = REF["predictor"][seed]
     L, E, cap = 6, 8, 12
     rng = np.random.default_rng(seed)
-    lib = _library(rng, 9, L, E)
-    with _cpu_only_torch():
-        ns.expert_tracer.ExpertTracer._instance = None
-        rt = ns.expert_tracer.ExpertTracer(cap, _cfg(L, E))
-        rt.trace_collection[:9] = torch.from_numpy(lib)
-        rp = ns.expert_predictor.ExpertPredictor(_cfg(L, E))
-        rp.add_tracer(rt)
-        ot = M.ExpertTracer(cap, L, E)
-        ot.load_trace(lib)
-        op = M.ExpertPredictor(L, E)
-        op.add_tracer(ot)
-        rs, os_ = rt.create_entry(), ot.create_entry()
-        for step in range(3):
-            for layer in range(L):
-                experts = rng.integers(0, E, size=(4, 2))
-                a = rp.predict(rs, torch.from_numpy(experts), layer)
-                b = op.predict(os_, experts, layer)
-                np.testing.assert_allclose(a, b, rtol=1e-6, atol=1e-9)
-        np.testing.assert_array_equal(rt.get_entry(rs).matrix, ot.get_entry(os_).matrix)
-        np.testing.assert_array_equal(rt.collection_access, ot.collection_access)
+    lib = library(rng, 9, L, E)
+    ot = M.ExpertTracer(cap, L, E)
+    ot.load_trace(lib)
+    op = M.ExpertPredictor(L, E)
+    op.add_tracer(ot)
+    os_ = ot.create_entry()
+    i = 0
+    for step in range(3):
+        for layer in range(L):
+            experts = rng.integers(0, E, size=(4, 2))
+            b = op.predict(os_, experts, layer)
+            np.testing.assert_allclose(ref["predict"][i], b, rtol=1e-6, atol=1e-9)
+            i += 1
+    assert i == len(ref["predict"])
+    np.testing.assert_array_equal(ref["matrix"], ot.get_entry(os_).matrix)
+    np.testing.assert_array_equal(ref["collection_access"], ot.collection_access)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present (GPU box)")
 def test_prefetch_request_order_matches_literal_reference():
-    import ref_loader
-    ns = ref_loader.load()
+    ref = REF["prefetch"]
     L, E = 5, 4
-    rng = np.random.default_rng(3)
-    matrix = rng.random((L, E)) * (rng.random((L, E)) > 0.3)
+    matrix, tmap = prefetch_inputs(L, E)
 
     class Rec:
         def __init__(self):
@@ -98,21 +56,13 @@ def test_prefetch_request_order_matches_literal_reference():
         def enqueue_prefetch(self, tid, gpu):
             self.enq.append(tid)
 
-    tmap = {(l, e): 100 + l * E + e for l in range(L) for e in range(E)}
-    import io, contextlib as cl
-    with cl.redirect_stdout(io.StringIO()):
-        rp = ns.expert_prefetcher.ExpertPrefetcher(_cfg(L, E))
-    rp.expert_tensor_map = tmap
-    r1 = Rec()
-    rp.set_archer_engine(r1)
-    rp.prefetch_experts(2, matrix)
     op = M.ExpertPrefetcher(L, E)
     op.expert_tensor_map = tmap
     r2 = Rec()
     op.set_archer_engine(r2)
     op.prefetch_experts(2, matrix)
-    assert r1.cands == r2.cands and r1.enq == r2.enq
-    assert [tmap[p] for p, _ in op.ordered_requests(2, matrix)] == r1.enq
+    assert ref["cands"] == r2.cands and ref["enq"] == r2.enq
+    assert [tmap[p] for p, _ in op.ordered_requests(2, matrix)] == ref["enq"]
 
 
 def test_degenerate_empty_library_prefetches_everything_nearest_first():
@@ -140,26 +90,11 @@ def test_tracer_finish_entry_and_counts():
     assert tr.trace_collection[0].sum() == 6 and tr.collection_access[0] == 1
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("current_layer", [0, 2, 3, 5])
+@pytest.mark.parametrize("current_layer", PRIORITY_LAYERS)
 def test_priority_score_matches_literal_reference(current_layer):
-    import importlib
-    import ref_loader
-    ref_loader.load()
-    ps = importlib.import_module("moe_infinity.memory.expert_priority_score")
-    ent = importlib.import_module("moe_infinity.memory.expert_entry")
-    L, E = 6, 4
-    rng = np.random.default_rng(current_layer)
-    dec = rng.integers(0, 4, size=(L, E)).astype(np.float64)
-    dec[1] = 0                                           # an all-zero layer row
-    freq = {(int(e), int(l)): float(rng.integers(0, 5)) for l in range(L) for e in range(E) if rng.random() < 0.6}
-    entry = ent.ExpertTraceEntry("s", dec.copy(), 0, 0)
-    ref_list = ps.priority_score(freq, set(), set(), entry, current_layer, L)
-    ref_m = np.zeros((L, E))
-    for ce in ref_list:
-        ref_m[ce.layer_idx, ce.expert_idx] = ce.r
+    L, E, dec, freq = priority_inputs(current_layer)
     ours = M.priority_score_matrix(freq, dec, current_layer, L)
-    np.testing.assert_allclose(ours, ref_m, rtol=1e-12, atol=0)
+    np.testing.assert_allclose(ours, REF["priority_score"][current_layer], rtol=1e-12, atol=0)
 
 
 # ---------------------------------------------------------------- cache policy oracle: the stated rules

@@ -2,9 +2,9 @@
 
   * test_oracle_matches_reference_golden: always runs; tests/golden/expert_ffn_ref.pt was produced by
     /root/reference/core/parallel/expert_module.cpp compiled as-is (tests/golden/make_expert_golden.py).
-  * test_oracle_matches_live_reference_module: runs wherever oracle/_ref/ref_expert_module.so exists (the dev
-    container builds it in __graft_entry__.build(); the file travels to the GPU box) on fresh random shapes.
-Bit equality is demanded: both sides call the same ATen operators on the same CPU.
+  * test_oracle_matches_live_reference_module: the same module on seeded random shapes of every expert type and dtype;
+    tests/golden/expert_ffn_live_ref.pt holds its outputs (tests/golden/make_reference_golden.py).
+Bit equality is demanded: both sides call the same ATen operators on the CPU.
 """
 from __future__ import annotations
 
@@ -19,9 +19,10 @@ sys.path.insert(0, os.path.join(HERE, "golden"))
 
 import expert_cases as C  # noqa: E402
 from oracle import moe_oracle as O  # noqa: E402
-from oracle import ref_module  # noqa: E402
+from reference_cases import SHAPES, rand_case, seed_of  # noqa: E402
 
 GOLD = torch.load(os.path.join(HERE, "golden", "expert_ffn_ref.pt"))
+LIVE = torch.load(os.path.join(HERE, "golden", "expert_ffn_live_ref.pt"))
 
 
 @pytest.mark.parametrize("name", sorted(C.CASES))
@@ -36,31 +37,15 @@ def test_oracle_matches_reference_golden(name):
     assert torch.equal(y, g["y"]), f"{name}: max |diff| {(y.float() - g['y'].float()).abs().max()}"
 
 
-def _rand_case(et, dt, H, I, n, seed):
-    g = torch.Generator().manual_seed(seed)
-    r = lambda *s: (torch.randn(*s, generator=g) * 0.1).to(dt)  # noqa: E731
-    if et == 0:
-        ws = [r(I, H), r(H, I)]
-    elif et == 4:
-        ws = [r(I, H), r(H, I), r(I, H)]
-    elif et in (1, 5):
-        ws = [r(I, H), r(I, H), r(H, I)]
-    else:
-        ws = [r(I, H), r(I), r(H, I), r(H)]
-    return ws, torch.randn(n, H, generator=g).to(dt)
-
-
 @pytest.mark.parametrize("et", [0, 1, 2, 3, 4, 5])
 @pytest.mark.parametrize("di", [0, 1, 2])
 def test_oracle_matches_live_reference_module(et, di):
-    R = ref_module.load()
-    if R is None:
-        pytest.skip("oracle/_ref/ref_expert_module.so not built (needs /root/reference at build time)")
     torch.set_num_threads(1)
     dt = C.DT[di]
-    for i, (H, I, n) in enumerate([(32, 48, 1), (64, 40, 13), (72, 136, 4), (256, 512, 33)]):
-        ws, x = _rand_case(et, dt, H, I, n, 1000 + 17 * et + 5 * di + i)
-        y_ref = R.expert_forward(et, di, ws, x)
+    assert len(LIVE[(et, di)]) == len(SHAPES)
+    for i, (H, I, n) in enumerate(SHAPES):
+        ws, x = rand_case(et, dt, H, I, n, seed_of(et, di, i))
+        y_ref = LIVE[(et, di)][i]
         y = O.expert_ffn(x, ws, et)
         assert y.dtype == y_ref.dtype
         assert torch.equal(y, y_ref), f"type {et} dtype {dt} shape {(H, I, n)}"
@@ -68,9 +53,8 @@ def test_oracle_matches_live_reference_module(et, di):
 
 def test_switch_module_casts_weights_to_input_dtype():
     """expert_module.cpp:31-35: fp32 weights, bf16 activations -> weights are cast per call."""
-    R = ref_module.load()
-    if R is None:
-        pytest.skip("oracle/_ref not built")
-    ws, x = _rand_case(0, torch.float32, 64, 96, 6, 77)
+    ws, x = rand_case(0, torch.float32, 64, 96, 6, 77)
     xb = x.to(torch.bfloat16)
-    assert torch.equal(O.expert_ffn(xb, ws, 0), R.expert_forward(0, 1, ws, xb))
+    y_ref = LIVE["switch_cast"]
+    assert y_ref.dtype == torch.bfloat16
+    assert torch.equal(O.expert_ffn(xb, ws, 0), y_ref)

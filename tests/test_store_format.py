@@ -2,8 +2,9 @@
 
   * golden: tests/golden/archer_index_ref.bin was written by `ArcherTensorIndex::Serialize`
     (core/aio/archer_tensor_index.cpp:105-113 compiled as-is, tests/golden/make_store_golden.py) -- always checked;
-  * live (wherever oracle/_ref/ref_expert_module.so exists): our writer -> the reference's `Deserialize`, the reference's
-    `Serialize` -> our parser, on random tensor sets;
+  * round trip on random tensor sets: our writer -> the reference's `Deserialize`, the reference's `Serialize` -> our
+    parser (what the reference code read and wrote is recorded in tests/golden/reference_results.pt by
+    tests/golden/make_reference_golden.py; our writer must still produce the bytes it read);
   * the data files: 4096-byte aligned offsets (kAioAlignment), whole aligned blocks on disk, StoreTensor's rules for
     known ids, reload, expert blobs, and the opt-in persistent mode of compat.prefetch_handle.
 Bit-exact: it is a byte format."""
@@ -19,9 +20,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 
 from make_store_golden import STORE_GOLDEN_ENTRIES  # noqa: E402
+from reference_cases import STORE_SEEDS, random_tensors  # noqa: E402
 from moe_infinity_b200.store import ALIGN, ArcherTensorStore, TensorMeta, parse_index, serialize_index  # noqa: E402
-from oracle import ref_module  # noqa: E402
 
+REF = torch.load(os.path.join(HERE, "golden", "reference_results.pt"), weights_only=False)["store"]
 _SCALAR = {torch.uint8: 0, torch.int64: 4, torch.float16: 5, torch.float32: 6, torch.bfloat16: 15, torch.float8_e4m3fn: 24}
 
 
@@ -47,43 +49,26 @@ def test_parser_reads_the_reference_writers_file():
             parse_index(bad)
 
 
-def _random_tensors(seed, n):
-    g = torch.Generator().manual_seed(seed)
-    dts = [torch.bfloat16, torch.float16, torch.float32, torch.int64, torch.uint8, torch.bool, torch.float64]
-    out = {}
-    for i in range(n):
-        dt = dts[int(torch.randint(0, len(dts), (1,), generator=g))]
-        rank = int(torch.randint(0, 4, (1,), generator=g))
-        shape = [int(torch.randint(1, 40, (1,), generator=g)) for _ in range(rank)]
-        t = (torch.randn(shape, generator=g) * 10)
-        t = (t > 0) if dt == torch.bool else t.to(dt)
-        out[int(torch.randint(0, 2 ** 31, (1,), generator=g)) * 2 + (i % 2)] = t
-    return out
-
-
 def test_round_trip_with_the_compiled_reference_index_code(tmp_path):
-    R = ref_module.load()
-    if R is None:
-        pytest.skip("oracle/_ref/ref_expert_module.so not built (needs /root/reference at build time)")
-    for seed in range(4):
-        tensors = _random_tensors(seed, 25)
+    for seed in STORE_SEEDS:
+        ref = REF[seed]
+        tensors = random_tensors(seed, 25)
         d = tmp_path / f"s{seed}"
         store = ArcherTensorStore(str(d))
         for tid, t in tensors.items():
             store.store_tensor(tid, t, flush=False)
         store.flush()
-        # ours -> reference reader
-        got = {e[0]: e[1:] for e in R.index_deserialize(store.index_path)}
+        # ours -> reference reader: the file is the one the reader read, and what it read is what we meant
+        with open(store.index_path, "rb") as f:
+            assert f.read() == ref["our_index"]
+        got = ref["ref_deserialize"]
         assert sorted(got) == sorted(tensors)
         for tid, t in tensors.items():
             m = store.index[tid]
             assert got[tid] == (m.file_id, m.offset, t.numel() * t.element_size(), list(t.shape), m.scalar_type, 0, -1, 0,
                                 False, False)
         # reference writer -> ours (same metas, built by the reference from the tensors themselves)
-        ref_path = str(d / "ref_index")
-        R.index_serialize(ref_path, [(tid, store.index[tid].file_id, store.index[tid].offset, t) for tid, t in tensors.items()])
-        with open(ref_path, "rb") as f:
-            assert parse_index(f.read()) == store.index
+        assert parse_index(ref["ref_index"]) == store.index
 
 
 def test_data_file_layout_and_store_rules(tmp_path):
